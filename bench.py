@@ -23,6 +23,8 @@ source.  One JSON line on stdout:
                 only place that touches oracle/; the package never does)
 
 `--impl reference` times the reference's CPU implementation instead (rank 0 only).
+`--dump-outputs DIR` also writes what the last timed step computed to DIR/*.npy
+(levels / distances / ranks, or the triangle count; see dump_outputs).
 """
 import argparse
 import json
@@ -63,7 +65,16 @@ def parse_args():
     ap.add_argument("--edgefactor", type=int, default=16)
     ap.add_argument("--seed", type=int, default=1)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step "
+                         "computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "ours" or args.gpus != 1 or
+                                          int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs writes the results of the single-GPU path: "
+                 "use it with --impl ours --gpus 1 in a single process")
     if args.scale is None:
         env = os.environ.get("GB200_BENCH_SCALE")
         args.scale = int(env) if env else DEFAULT_SCALE[args.algo]
@@ -400,6 +411,40 @@ def workload_config(args, n, nnz, source):
             "partition": "1-D row slices" if args.gpus > 1 else "single GPU"}
 
 
+# --dump-outputs: the result a caller of the timed path receives, one float32 or
+# float64 .npy file per array.  A vector longer than DUMP_SAMPLE entries is written
+# as a fixed sample (DUMP_SEED) of DUMP_SAMPLE entries in index order, with the
+# sampled indices in <name>_index.npy, which keeps the files under DUMP_LIMIT bytes
+# in all.  The inputs depend on the arguments only, so two builds of the library
+# run with the same arguments can be compared entry for entry.
+DUMP_NAMES = {"bfs": "levels", "sssp": "distances", "pr": "ranks"}
+DUMP_SAMPLE = 1 << 22
+DUMP_SEED = 1
+DUMP_LIMIT = 64 * 10**6
+
+
+def dump_outputs(out_dir, outputs):
+    """outputs: name -> 1-D array; written as out_dir/<name>.npy."""
+    import numpy as np
+    files = {}
+    for name, a in outputs.items():
+        a = np.asarray(a)
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        if a.size > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(
+                a.size, DUMP_SAMPLE, replace=False))
+            files[name + "_index"] = idx.astype(np.float64)
+            a = a[idx]
+        files[name] = a
+    total = sum(a.nbytes for a in files.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit"
+                           % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in files.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 KINDS = ["spmvMergeKernel / spmvHubKernel (generic pull SpMV)",
          "spmvMaskedOrPullKernel (fused Boolean pull)",
          "spmspvPushKernel (push SpMSpV expand)",
@@ -555,6 +600,13 @@ def main():
         if st[0] > 0:
             fused_stats = [int(x) for x in st]
             KINDS[1] = "bfsFusedKernel (whole traversal: Boolean pull + push levels)"
+    if args.dump_outputs is not None:
+        # before the end-to-end runs below overwrite the result
+        if args.algo == "tc":
+            dump_outputs(args.dump_outputs, {"triangles": [tc_count[0]]})
+        else:
+            dump_outputs(args.dump_outputs,
+                         {DUMP_NAMES[args.algo]: result_vec.extractTuples()})
     dom = max(range(4), key=lambda k: prof[k][0])
     peak, peak_src = measured_peak_hbm()
     dom_ms, dom_launches, dom_bytes = prof[dom]

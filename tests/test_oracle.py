@@ -2,7 +2,9 @@
   (1) the committed golden vectors generated from the reference's own CPU code
       (tests/golden/golden.json, tests/golden/make_golden.py),
   (2) the known answers pinned by the reference's tests/fixtures (BASELINE.md §2),
-  (3) oracle/_ref/libgbref.so itself, when it is present in this checkout.
+  (3) what the reference's own CPU code (oracle/_ref/libgbref.so) returns on the
+      same inputs, stored in tests/golden/ref_cpu.npz
+      (tests/golden/make_golden_ref.py).
 """
 import json
 import os
@@ -14,6 +16,7 @@ import oracle_binding as orc
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLDEN = json.load(open(os.path.join(HERE, "golden", "golden.json")))
+REF_CPU = np.load(os.path.join(HERE, "golden", "ref_cpu.npz"))
 
 CHESAPEAKE_LEVELS = [1, 3, 3, 3, 3, 3, 2, 2, 3, 3, 2, 2, 2, 3, 3, 3, 3, 3, 3, 3,
                      3, 2, 2, 3, 3, 3, 3, 3, 3, 3, 3, 3, 3, 2, 2, 3, 2, 3, 2]
@@ -175,25 +178,27 @@ def test_weight_stream_golden():
     assert got.min() >= 1 and got.max() <= 64
 
 
-needs_ref = pytest.mark.skipif(orc.ref() is None,
-                               reason="oracle/_ref not built in this checkout")
+def colind_checksum(ci):
+    return int(np.sum(ci.astype(np.int64) * (np.arange(len(ci), dtype=np.int64) % 97 + 1)))
 
 
-@needs_ref
 @pytest.mark.parametrize("scale", [8, 12])
 def test_oracle_equals_reference_cpu_on_rmat(scale):
+    ref = {k[len("rmat%d_" % scale):]: REF_CPU[k] for k in REF_CPU.files
+           if k.startswith("rmat%d_" % scale)}
     rp, ci = orc.rmat_csr(scale)
+    assert len(ci) == ref["nnz"] and colind_checksum(ci) == ref["colind_checksum"]
     src = int(np.argmax(np.diff(rp)))
-    assert np.array_equal(orc.bfs(rp, ci, src), orc.ref_bfs(rp, ci, src))
-    assert np.array_equal(orc.bfs(rp, ci, 0), orc.ref_bfs(rp, ci, 0))
-    w = orc.ref_uniform_weights(1, 1, 64, len(ci))
-    assert np.array_equal(orc.sssp(rp, ci, w, src), orc.ref_sssp(rp, ci, w, src))
-    assert np.array_equal(orc.pr(rp, ci), orc.ref_pr(rp, ci))
+    assert src == ref["source"]
+    assert np.array_equal(orc.bfs(rp, ci, src), ref["bfs_source"])
+    assert np.array_equal(orc.bfs(rp, ci, 0), ref["bfs_0"])
+    w = ref["weights"].astype(np.float32)
+    assert np.array_equal(orc.sssp(rp, ci, w, src), ref["sssp_source"])
+    assert np.array_equal(orc.pr(rp, ci), ref["pr"])
     lr, lc = orc.tril(rp, ci)
-    assert orc.tc(lr, lc) == orc.ref_tc(lr, lc)
+    assert orc.tc(lr, lc) == ref["tc"]
 
 
-@needs_ref
 @pytest.mark.parametrize("name,directed", [("chesapeake.mtx", 2),
                                            ("chesapeake.mtx", 0),
                                            ("test_cc.mtx", 0),
@@ -208,35 +213,39 @@ def test_loader_equals_reference_readmtx(name, directed):
     n, src, dst, symmetric = orc.read_mtx_edges(path)
     undirected = (symmetric or directed == 2) and directed != 1
     rp, ci = orc.build_csr(n, src, dst, undirected)
-    rr, rc, _ = orc.ref_load_mtx(path, directed)
-    assert np.array_equal(rp, rr) and np.array_equal(ci, rc)
+    key = "mtx_%s_d%d_" % (os.path.splitext(name)[0], directed)
+    assert np.array_equal(rp, REF_CPU[key + "rowptr"])
+    assert np.array_equal(ci, REF_CPU[key + "colind"])
 
 
-@needs_ref
 def test_oracle_equals_reference_cpu_on_random_graphs():
-    """Property test of the oracle pin: on random undirected graphs of assorted
-    shapes (isolated vertices, multi-edges in the input, tiny and ragged degrees)
-    the restatement and the reference's own CPU code agree bit for bit on BFS,
-    SSSP, PageRank and the triangle count."""
-    from hypothesis import given, settings, strategies as st
+    """Property test of the oracle pin: on 100 random undirected graphs of assorted
+    shapes (isolated vertices, multi-edges in the input, tiny and ragged degrees;
+    fixed draws, edge cases first) the restatement agrees bit for bit with the
+    reference's own CPU code on BFS, SSSP, PageRank and the triangle count."""
+    cases = REF_CPU["rand_cases"]
+    assert len(cases) == 100
+    n_all, nnz_all = cases[:, 0], REF_CPU["rand_nnz"]
 
-    @settings(max_examples=60, deadline=None)
-    @given(n=st.integers(2, 60), m=st.integers(0, 400), seed=st.integers(0, 2**31 - 1))
-    def check(n, m, seed):
+    def per_case(key, sizes):
+        return np.split(REF_CPU["rand_" + key], np.cumsum(sizes)[:-1])
+    bfs_0, bfs_last, pr = (per_case(k, n_all) for k in ("bfs_0", "bfs_last", "pr"))
+    weights = per_case("weights", nnz_all)
+    sssp_0 = per_case("sssp_0", np.where(nnz_all > 0, n_all, 0))
+    for i, (n, m, seed) in enumerate(cases.tolist()):
         rng = np.random.RandomState(seed)
         src = rng.randint(0, n, m).astype(np.int32)
         dst = rng.randint(0, n, m).astype(np.int32)
         rp, ci = orc.build_csr(n, src, dst, True)          # drops loops/duplicates
-        for s in (0, n - 1):
-            assert np.array_equal(orc.bfs(rp, ci, s), orc.ref_bfs(rp, ci, s))
+        assert len(ci) == nnz_all[i]
+        assert np.array_equal(orc.bfs(rp, ci, 0), bfs_0[i])
+        assert np.array_equal(orc.bfs(rp, ci, n - 1), bfs_last[i])
         if len(ci):
-            w = orc.ref_uniform_weights(seed % 1000, 1, 64, len(ci))
-            assert np.array_equal(orc.sssp(rp, ci, w, 0), orc.ref_sssp(rp, ci, w, 0))
-        assert np.array_equal(orc.pr(rp, ci), orc.ref_pr(rp, ci))
+            w = weights[i].astype(np.float32)
+            assert np.array_equal(orc.sssp(rp, ci, w, 0), sssp_0[i])
+        assert np.array_equal(orc.pr(rp, ci), pr[i])
         lr, lc = orc.tril(rp, ci)
-        assert orc.tc(lr, lc) == orc.ref_tc(lr, lc)
-
-    check()
+        assert orc.tc(lr, lc) == REF_CPU["rand_tc"][i]
 
 
 @pytest.mark.parametrize("scale", [14, 16])

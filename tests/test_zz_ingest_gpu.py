@@ -1,6 +1,6 @@
 """Device ingest (SURVEY.md §8 f1): the library's own radix sort, tuples -> CSR with
 the reference loader's semantics, CSR -> CSC, and the Matrix Market path, against
-numpy, the oracle and the reference's own loader (oracle/_ref)."""
+numpy, the oracle and the reference's own loader (oracle/_ref, stored results)."""
 import ctypes as C
 import os
 
@@ -113,17 +113,19 @@ def test_csr_transpose_values(gb):
                                            ("test_bc.mtx", 2)])
 def test_matrix_market_path_matches_the_reference_loader(gb, name, directed):
     """gb200_matrix_load_mtx parses on the host and orders / symmetrises / dedups on
-    the device; the CSR must be the reference readMtx + coo2csr's (oracle/_ref).
+    the device; the CSR must be the reference readMtx + coo2csr's (oracle/_ref, as
+    stored in tests/golden/ref_cpu.npz by tests/golden/make_golden_ref.py).
     test_sgm.mtx (nothing but self-loops) is left out: the reference's removeSelfloop
     (util.hpp:310-322) reads past the end of its vectors when every tuple is dropped,
     and depending on what the heap holds it returns or dies in vector::resize(-1); the
     all-loops case is covered in test_ingest_edge_cases."""
-    if orc.ref() is None:
-        pytest.skip("oracle/_ref not built")
     path = os.path.join(GOLDEN, name)
     A = gb.Matrix.from_mtx(path, directed=directed)
     rp, ci, val = A.extract_csr()
-    want_rp, want_ci, want_val = orc.ref_load_mtx(path, directed)
+    key = "mtx_%s_d%d_" % (os.path.splitext(name)[0], directed)
+    with np.load(os.path.join(GOLDEN, "ref_cpu.npz")) as ref:
+        want_rp, want_ci, want_val = (ref[key + "rowptr"], ref[key + "colind"],
+                                      ref[key + "val"])
     assert np.array_equal(rp, want_rp)
     assert np.array_equal(ci, want_ci)
     assert np.array_equal(val, want_val)
