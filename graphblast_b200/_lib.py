@@ -108,7 +108,6 @@ SIGNATURES = [
     ("gb200_xchg_free", _I, [_P]),
     ("gb200_xchg_allgather_bits", _I, [_P, _P, C.POINTER(_LL)]),
     ("gb200_xchg_bits_ptr", _I, [_P, C.POINTER(_P)]),
-    ("gb200_dist_bfs", _I, [_P, _P, _P, _LL, _LL, _P, C.POINTER(_I)]),
     ("gb200_dist_bfs_fused", _I, [_P, _P, _P, _LL, _LL, _P, C.POINTER(_I)]),
     ("gb200_xchg_allgather_words", _I, [_P, _P, _D, C.POINTER(_D)]),
     ("gb200_dist_pr", _I, [_P, _P, _P, _LL, _F, _F, _P, C.POINTER(_I)]),

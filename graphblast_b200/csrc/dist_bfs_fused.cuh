@@ -6,7 +6,7 @@
 //   flags2[world]         flags2[r] = (last epoch rank r has published << 32) | size of
 //                         the slice it published
 //
-// The host-loop form (gb200_dist_bfs) pays per level: bitmap export, publish kernel,
+// A level loop on the host (r01) paid per level: bitmap export, publish kernel,
 // one-warp wait kernel, a host mailbox read, OR / import passes and the generic
 // assign + mxv launches — about 40 us of latency against 10..100 us of work, which
 // is why two GPUs were slower than one in r01.  Here a level is:
@@ -15,7 +15,7 @@
 //                 replicated visited bitmap; heavy columns by the whole grid.
 //                 pull: every owned unvisited row probes the replicated visited
 //                 bitmap (first-neighbour summary, early exit) — operand reuse in
-//                 its global form, as in gb200_dist_bfs.
+//                 its global form (reference kernels/spmv.hpp:36-38).
 //   publish       all threads store the owned slice of the new frontier into
 //                 data[epoch & 1] of EVERY rank (peer stores), then one thread
 //                 writes this rank's count and flag to every rank and spins on the
@@ -349,7 +349,7 @@ bfsFusedDistKernel(BfsDistArgs a) {
 
 extern "C" {
 
-// Same contract as gb200_dist_bfs (dist_exchange.cuh), one cooperative launch.
+// Contract in include/graphblast_b200.h; one cooperative launch per traversal.
 int gb200_dist_bfs_fused(gb200_xchg_t x, gb200_vector_t v, gb200_matrix_t M,
                          long long n, long long source, gb200_desc_t desc,
                          int* levels_out) {
@@ -404,9 +404,7 @@ int gb200_dist_bfs_fused(gb200_xchg_t x, gb200_vector_t v, gb200_matrix_t M,
   a.epoch0 = x->epoch;
   a.timeout_cycles = 20000000000ll;
 
-  static const int minb = getEnv("GB200_BFS_MINB", 2);
-  void (*kernel)(gbx::BfsDistArgs) = (minb >= 2) ? gbx::bfsFusedDistKernel<2>
-                                                 : gbx::bfsFusedDistKernel<1>;
+  void (*kernel)(gbx::BfsDistArgs) = gbx::bfsFusedDistKernel<2>;
   static int resident = 0;
   if (resident == 0) {
     int per_sm = 0;

@@ -1,5 +1,6 @@
 // graphblast_b200 — multi-GPU frontier exchange over peer memory and the native
-// level loop of the 1-D row-partitioned BFS (SURVEY.md §8e).  Included by capi.cu.
+// loops of the 1-D row-partitioned PageRank and SSSP (SURVEY.md §8e); the BFS is
+// dist_bfs_fused.cuh.  Included by capi.cu.
 //
 // One process per GPU.  Every rank owns a block of device memory that all ranks
 // map through CUDA IPC:
@@ -30,13 +31,8 @@ struct gb200_xchg_s {
   char** d_peer;                         // device copy of peer[]
   unsigned long long  epoch;             // publishes issued so far
   unsigned long long* d_cells;           // [0] finished CTAs, [1] popcount, [2] total
-  unsigned int*       d_visited;         // cumulative visited bitmap (total_words)
   unsigned int*       d_seed;            // owned-slice scratch
   bool connected;
-  // vectors of the level loop, kept across traversals
-  graphblas::Vector<float>* f_own;
-  graphblas::Vector<float>* f2;
-  graphblas::Vector<float>* f_glob;
   // vectors of the PageRank loop: p_glob, p_prev_own, p_swap, r, r_temp
   graphblas::Vector<float>* pr_vec[5];
   // vectors of the SSSP loop: frontier_glob (view), relaxed, improved
@@ -168,18 +164,6 @@ __global__ void xchgWaitKernel(const char* __restrict__ local, size_t off_counts
   }
 }
 
-// dst[i] |= src[i]
-__global__ void orWordsKernel(unsigned int* __restrict__ dst,
-                              const unsigned int* __restrict__ src, size_t n) {
-  size_t i = static_cast<size_t>(blockIdx.x)*blockDim.x + threadIdx.x;
-  const size_t stride = static_cast<size_t>(gridDim.x)*blockDim.x;
-  for (; i < n; i += stride) dst[i] |= src[i];
-}
-
-__global__ void setBitKernel(unsigned int* words, long long bit) {
-  words[bit >> 5] = 1u << (bit & 31);
-}
-
 inline int publish(gb200_xchg_s* x, const unsigned int* d_words,
                    const unsigned long long* d_count, int use_imm = 0,
                    unsigned long long imm = 0ull) {
@@ -258,7 +242,6 @@ int gb200_xchg_create(gb200_xchg_t* out, int world, int rank,
   CUDA_CALL(cudaMemset(x->local, 0, x->bytes));
   CUDA_CALL(cudaMalloc(&x->d_cells, 8*sizeof(unsigned long long)));
   CUDA_CALL(cudaMemset(x->d_cells, 0, 8*sizeof(unsigned long long)));
-  CUDA_CALL(cudaMalloc(&x->d_visited, (x->total_words + 8)*4));
   CUDA_CALL(cudaMalloc(&x->d_seed, (x->total_words + 8)*4));
   CUDA_CALL(cudaMalloc(&x->d_peer, world*sizeof(char*)));
   x->peer.assign(world, static_cast<char*>(NULL));
@@ -268,7 +251,6 @@ int gb200_xchg_create(gb200_xchg_t* out, int world, int rank,
   if (world == 1)
     CUDA_CALL(cudaMemcpy(x->d_peer, x->peer.data(), sizeof(char*),
         cudaMemcpyHostToDevice));
-  x->f_own = NULL; x->f2 = NULL; x->f_glob = NULL;
   for (int i = 0; i < 5; ++i) x->pr_vec[i] = NULL;
   for (int i = 0; i < 3; ++i) x->ss_vec[i] = NULL;
   *out = x;
@@ -312,9 +294,8 @@ int gb200_xchg_free(gb200_xchg_t x) {
   cudaDeviceSynchronize();
   for (int p = 0; p < x->world; ++p)
     if (p != x->rank && x->peer[p] != NULL) cudaIpcCloseMemHandle(x->peer[p]);
-  cudaFree(x->local); cudaFree(x->d_cells); cudaFree(x->d_visited);
+  cudaFree(x->local); cudaFree(x->d_cells);
   cudaFree(x->d_seed); cudaFree(x->d_peer);
-  delete x->f_own; delete x->f2; delete x->f_glob;
   for (int i = 0; i < 5; ++i) delete x->pr_vec[i];
   for (int i = 0; i < 3; ++i) delete x->ss_vec[i];
   delete x;
@@ -342,107 +323,6 @@ int gb200_xchg_bits_ptr(gb200_xchg_t x, const uint32_t** d_bits) {
   if (x == NULL || d_bits == NULL) return rc(graphblas::GrB_NULL_POINTER);
   *d_bits = gbx::current(x);
   return 0;
-}
-
-// Level-synchronous BFS over the 1-D row partition, host loop in C++:
-//   v    (length nl = owned vertices)  levels of the owned vertices (output)
-//   M    nl x n local matrix: CSR rows = owned destinations (pull), CSC = the
-//        same entries by global source column (push)
-// Per level: v<f_own> = level;  f2<!v> = M (||.&&) u  with u = the cumulative
-// visited set when pulling (any visited neighbour discovers an unvisited row —
-// the operand-reuse shortcut of reference kernels/spmv.hpp:36-38 in its global
-// form) and u = the frontier when pushing;  all ranks exchange f2 through peer
-// memory.  The direction follows the frontier ratio with the hysteresis of
-// reference vector.hpp:318-342.
-int gb200_dist_bfs(gb200_xchg_t x, gb200_vector_t v, gb200_matrix_t M,
-                   long long n, long long source, gb200_desc_t desc,
-                   int* levels_out) {
-  if (x == NULL || v == NULL || M == NULL || desc == NULL)
-    return rc(graphblas::GrB_NULL_POINTER);
-  if (!x->connected || M->f == NULL) return rc(graphblas::GrB_UNINITIALIZED_OBJECT);
-  GB200_REQUIRE_DEVICE();
-  using namespace graphblas;          // NOLINT(build/namespaces)
-  using graphblas::backend::gbStream;
-  using graphblas::backend::gridFor;
-  cudaStream_t s = gbStream();
-  Descriptor* d = &desc->desc;
-  const size_t w_lo = x->word_off[x->rank];
-  const size_t nw   = x->word_off[x->rank + 1] - w_lo;
-  Index nl;
-  CHECK(v->f->size(&nl));
-  const long long lo = static_cast<long long>(w_lo)*32;
-  if (x->f_own == NULL) {
-    x->f_own  = new Vector<float>(nl);
-    x->f2     = new Vector<float>(nl);
-    x->f_glob = new Vector<float>(static_cast<Index>(n));
-  }
-  gb200_vector_s own_h  = {GB200_FP32, x->f_own};
-  gb200_vector_s f2_h   = {GB200_FP32, x->f2};
-  gb200_vector_s glob_h = {GB200_FP32, x->f_glob};
-
-  CHECK(v->f->fill(0.f));
-  CUDA_CALL(cudaMemsetAsync(x->d_visited, 0, x->total_words*4, s));
-  // level-1 frontier = {source}, published by its owner
-  CUDA_CALL(cudaMemsetAsync(x->d_seed, 0, (nw + 1)*4, s));
-  const bool own_src = source >= lo && source < lo + static_cast<long long>(nl);
-  if (own_src) {
-    gbx::setBitKernel<<<1, 1, 0, s>>>(x->d_seed, source - lo);
-    GB_KERNEL_CHECK();
-  }
-  CUDA_CALL(cudaMemsetAsync(x->d_cells + 3, 0, 8, s));
-  if (own_src) {
-    const unsigned long long one = 1ull;
-    CUDA_CALL(cudaMemcpyAsync(x->d_cells + 3, &one, 8, cudaMemcpyHostToDevice, s));
-  }
-  gbx::publish(x, x->d_seed, x->d_cells + 3);
-  long long total = gbx::wait(x);
-  if (total < 0) return rc(GrB_PANIC);
-
-  Desc_value saved_mode;
-  CHECK(d->get(GrB_MXVMODE, &saved_mode));
-  const float switchpoint = d->descriptor_.switchpoint();
-  float prev_ratio = 0.f;
-  bool  pulling = false;
-  int   level = 0;
-  Info  info = GrB_SUCCESS;
-  while (total > 0) {
-    ++level;
-    const unsigned int* gbits = gbx::current(x);
-    gbx::orWordsKernel<<<gridFor(x->total_words, 256), 256, 0, s>>>(
-        x->d_visited, gbits, x->total_words);
-    GB_KERNEL_CHECK();
-    // v<f_own> = level
-    if (gb200_vector_import_bits(&own_h, gbits + w_lo, -1) != 0) { info = GrB_PANIC; break; }
-    info = graphblas::assign<float, float, float, Index>(v->f, x->f_own,
-        GrB_NULL, static_cast<float>(level), GrB_ALL, nl, d);
-    if (info != GrB_SUCCESS) break;
-    // direction
-    const float ratio = static_cast<float>(total)/static_cast<float>(n);
-    if (!pulling) { if (ratio > switchpoint && ratio > prev_ratio) pulling = true; }
-    else          { if (ratio <= switchpoint && ratio < prev_ratio) pulling = false; }
-    prev_ratio = ratio;
-    if (pulling) {
-      if (gb200_vector_import_bits(&glob_h, x->d_visited, -1) != 0) { info = GrB_PANIC; break; }
-      CHECK(d->set(GrB_MXVMODE, GrB_PULLONLY));
-      CHECK(x->f2->vector_.setStorage(GrB_DENSE));
-    } else {
-      if (gb200_vector_import_bits(&glob_h, gbits, total) != 0) { info = GrB_PANIC; break; }
-      CHECK(d->set(GrB_MXVMODE, GrB_PUSHONLY));
-    }
-    CHECK(d->toggle(GrB_MASK));
-    info = graphblas::mxv<float, float, float, float>(x->f2, v->f, GrB_NULL,
-        LogicalOrAndSemiring<float>(), M->f, x->f_glob, d);
-    CHECK(d->toggle(GrB_MASK));
-    if (info != GrB_SUCCESS) break;
-    // the publish kernel counts the bits it sends
-    if (gb200_vector_export_bits(&f2_h, x->d_seed, NULL) != 0) { info = GrB_PANIC; break; }
-    gbx::publish(x, x->d_seed, NULL);
-    total = gbx::wait(x);
-    if (total < 0) { info = GrB_PANIC; break; }
-  }
-  d->set(GrB_MXVMODE, saved_mode);
-  if (levels_out != NULL) *levels_out = level;
-  return rc(info);
 }
 
 // Generic form for 32-bit payloads (float vectors): publishes nwords_owned words

@@ -84,9 +84,8 @@ Info bfsFused(Vector<float>* v, const Matrix<a>* A, Index s, Descriptor* desc, i
   args.counters   = reinterpret_cast<unsigned long long*>(base + 4*words_bytes);
   args.heavy      = reinterpret_cast<Index*>(base + 4*words_bytes + 256);
 
-  static const int minb = getEnv("GB200_BFS_MINB", 2);
   static int resident = 0;               // CTAs that fit at once (cooperative launch)
-  void (*kernel)(BfsFusedArgs) = (minb >= 2) ? bfsFusedKernel<GB_BFS_MINB> : bfsFusedKernel<1>;
+  void (*kernel)(BfsFusedArgs) = bfsFusedKernel<GB_BFS_MINB>;
   if (resident == 0) {
     int per_sm = 0;
     CUDA_CALL(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel,

@@ -20,39 +20,20 @@ Index compactOrdered(Source src, Index nitems, Descriptor* desc) {
   const int nblocks = static_cast<int>((nitems + per_cta - 1) / per_cta);
   unsigned long long* ctr = desc->counters() + 1;
   cudaStream_t s = gbStream();
-  // The single-launch look-back form is opt-in: measured on B200 it ties the
-  // three-launch form on the sparse BFS frontiers (0.567 vs 0.554 ms per RMAT-24
-  // traversal) and loses badly on dense SSSP frontiers, where its coarse CTAs
-  // serialise the emit loops (408 us per launch at RMAT-24).
-  static const bool one_pass = getEnv("GB200_COMPACT_1PASS", 0) != 0;
-  if (one_pass) {
-    // one launch, look-back across CTAs (kernels/compact.cuh)
-    const int nb1 = static_cast<int>((static_cast<long long>(nitems) +
-        GB_COMPACT_NT*GB_COMPACT_IPT - 1) / (GB_COMPACT_NT*GB_COMPACT_IPT));
-    unsigned long long* state = desc->lookback(static_cast<size_t>(nb1) + 1);
-    desc->lookback_epoch_ = desc->lookback_epoch_ % 0x3ffffffeu + 1u;
-    compactOnePassKernel<<<nb1, GB_COMPACT_NT, 0, s>>>(src, nitems, state,
-        desc->lookback_epoch_, ctr);
-    GB_KERNEL_CHECK();
-    return static_cast<Index>(runtime().fetch(ctr));
-  }
   int* block_counts = reinterpret_cast<int*>(
       desc->scratch(GB_SCRATCH_BLOCKSUM, static_cast<size_t>(nblocks)*sizeof(int)));
   // count + (last CTA) scan of the per-CTA counts, then emit: two launches
   // The total is posted to the host mailbox by the count pass, so the host
   // learns it while the emit pass is still running.
-  static const bool use_mail = getEnv("GB200_MAILBOX", 1) != 0;
-  const unsigned long long ticket = use_mail ? runtime().mailTicket() : 0ull;
+  const unsigned long long ticket = runtime().mailTicket();
   compactCountScanKernel<<<nblocks, GB_COMPACT_NT, 0, s>>>(src, nitems,
       block_counts, nblocks, desc->counters() + 2, ctr,
-      use_mail ? runtime().mailSlot(0) : NULL, ticket);
+      runtime().mailSlot(0), ticket);
   GB_KERNEL_CHECK();
   compactEmitKernel<<<nblocks, GB_COMPACT_NT, 0, s>>>(src, nitems,
       block_counts);
   GB_KERNEL_CHECK();
-  if (use_mail)
-    return static_cast<Index>(runtime().mailWait(0, ticket, ctr));
-  return static_cast<Index>(runtime().fetch(ctr));
+  return static_cast<Index>(runtime().mailWait(0, ticket, ctr));
 }
 
 }  // namespace backend

@@ -38,7 +38,6 @@ enum ScratchSlot {
   GB_SCRATCH_VEC_A,       // generic n-sized temporaries
   GB_SCRATCH_VEC_B,
   GB_SCRATCH_CUB,         // cub temp storage
-  GB_SCRATCH_LOOKBACK,    // compaction: ticket cell + per-CTA look-back status
   GB_SCRATCH_BFS,         // fused BFS: visited x2, frontier, next bitmaps + cells
   GB_SCRATCH_NSLOTS
 };
@@ -198,24 +197,6 @@ class Descriptor {
     return slot_ptr_[slot];
   }
   size_t scratchSize(ScratchSlot slot) const { return slot_size_[slot]; }
-
-  // Look-back state of the single-pass compaction: cell 0 is a ticket counter
-  // that only ever grows, cells 1..nblocks hold (epoch, flag, value) words.  The
-  // block is zeroed when (re)allocated; afterwards nothing is ever reset — each
-  // launch uses a fresh epoch and the ticket base the host has kept count of.
-  unsigned long long* lookback(size_t nblocks) {
-    const size_t bytes = (nblocks + 1)*sizeof(unsigned long long);
-    if (bytes > slot_size_[GB_SCRATCH_LOOKBACK]) {
-      void* p = scratch(GB_SCRATCH_LOOKBACK, bytes);
-      CUDA_CALL(cudaMemsetAsync(p, 0, slot_size_[GB_SCRATCH_LOOKBACK], gbStream()));
-      lookback_epoch_  = 0;
-      lookback_ticket_ = 0;
-    }
-    return reinterpret_cast<unsigned long long*>(
-        slot_ptr_[GB_SCRATCH_LOOKBACK]);
-  }
-  unsigned int       lookback_epoch_ = 0;
-  unsigned long long lookback_ticket_ = 0;
 
   // Device counters: 64 x 8-byte cells, zero when first handed out.  Cell 2 is
   // the "finished CTAs" counter of the compaction's count pass, which leaves it

@@ -99,102 +99,6 @@ compactEmitKernel(Source src, Index nitems,
 }
 
 // ---------------------------------------------------------------------------
-// Single-pass form (decoupled look-back): one launch instead of three.
-//   state[0] = ticket counter, state[1] = finished-CTA counter (both return to 0
-//   at the end of every launch), state[2 + b] = status word of logical block b:
-//   bits 63..34 launch epoch, bits 33..32 flag, bits 31..0 value.
-// Logical block ids come from the ticket, so a CTA only ever waits for CTAs that
-// are already running; status words of older launches are recognised by their
-// epoch and never need clearing.
-// ---------------------------------------------------------------------------
-#define GB_COMPACT_IPT  8
-#define GB_LB_AGGREGATE 1ull    // value = this block's own count
-#define GB_LB_INCLUSIVE 2ull    // value = count of blocks 0..b
-
-template <typename Source>
-__global__ void __launch_bounds__(GB_COMPACT_NT)
-compactOnePassKernel(Source src, Index nitems,
-                     unsigned long long* __restrict__ state,
-                     unsigned int epoch,
-                     unsigned long long* __restrict__ total_out) {
-  __shared__ int s_scan[GB_COMPACT_NT/32 + 1];
-  __shared__ unsigned int s_bid;
-  __shared__ int s_prefix;
-  if (threadIdx.x == 0)
-    s_bid = static_cast<unsigned int>(atomicAdd(state, 1ull));
-  __syncthreads();
-  const unsigned int bid = s_bid;
-  // GB_COMPACT_IPT consecutive items per thread (blocked, so order is kept): the
-  // look-back chain is as long as the grid, so CTAs are made coarse.
-  const Index item0 = (static_cast<Index>(bid)*GB_COMPACT_NT + threadIdx.x)
-                      *GB_COMPACT_IPT;
-  int cnt[GB_COMPACT_IPT];
-  int c = 0;
-#pragma unroll
-  for (int j = 0; j < GB_COMPACT_IPT; ++j) {
-    cnt[j] = (item0 + j < nitems) ? src.count(item0 + j) : 0;
-    c += cnt[j];
-  }
-  int total;
-  const int excl = blockExclusiveScan<GB_COMPACT_NT>(c, s_scan, &total);
-
-  if (threadIdx.x < 32) {
-    const int lane = threadIdx.x;
-    volatile unsigned long long* status = state + 2;
-    const unsigned long long tag = static_cast<unsigned long long>(epoch) << 34;
-    int prefix = 0;
-    if (bid == 0) {
-      if (lane == 0)
-        status[0] = tag | (GB_LB_INCLUSIVE << 32) | static_cast<unsigned int>(total);
-    } else {
-      if (lane == 0)
-        status[bid] = tag | (GB_LB_AGGREGATE << 32) | static_cast<unsigned int>(total);
-      int look = static_cast<int>(bid) - 1;     // lane l inspects block look - l
-      while (true) {
-        const int idx = look - lane;
-        unsigned long long v = tag | (GB_LB_INCLUSIVE << 32);   // "before block 0"
-        if (idx >= 0) {
-          do { v = status[idx]; }
-          while (static_cast<unsigned int>(v >> 34) != epoch);
-        }
-        const bool inclusive = ((v >> 32) & 3ull) == GB_LB_INCLUSIVE;
-        const unsigned int incl_mask = __ballot_sync(GB_FULL_MASK, inclusive);
-        const int first_incl = __ffs(incl_mask) - 1;          // -1: none
-        const unsigned int contrib =
-            (first_incl < 0 || lane <= first_incl) ? static_cast<unsigned int>(v) : 0u;
-        prefix += static_cast<int>(__reduce_add_sync(GB_FULL_MASK, contrib));
-        if (first_incl >= 0) break;
-        look -= 32;
-      }
-      if (lane == 0)
-        status[bid] = tag | (GB_LB_INCLUSIVE << 32) |
-                      static_cast<unsigned int>(prefix + total);
-    }
-    if (lane == 0) {
-      s_prefix = prefix;
-      if (bid == gridDim.x - 1)
-        *total_out = static_cast<unsigned long long>(prefix + total);
-    }
-  }
-  __syncthreads();
-  int pos = s_prefix + excl;
-#pragma unroll
-  for (int j = 0; j < GB_COMPACT_IPT; ++j) {
-    if (cnt[j] > 0) { src.emit(item0 + j, pos); pos += cnt[j]; }
-    else if (item0 + j < nitems) src.finish(item0 + j);
-  }
-
-  // last CTA out resets the two counters for the next launch
-  if (threadIdx.x == 0) {
-    __threadfence();
-    if (atomicAdd(state + 1, 1ull) == gridDim.x - 1) {
-      state[0] = 0ull;
-      state[1] = 0ull;
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------
 // Sources
 // ---------------------------------------------------------------------------
 

@@ -1,11 +1,15 @@
 // graphblast_b200 backend — masked SpGEMM (dot-product formulation) used by
 // triangle counting: C(i,j) = add_k mul(A(i,k), B(k,j)) only for (i,j) in mask.
 //
-// Reference: spgemmMaskedKernel, kernels/spgemm.hpp:17-79 — one warp per mask
-// row, every lane binary-searches A(i,:)'s columns in B(:,j) for each mask entry.
-// Here: warps pull mask rows from a device work counter (skewed RMAT rows no
-// longer pin a statically assigned warp), and for every mask entry the SHORTER
-// of the two sorted lists is scanned while the longer one is searched.
+// These are the search kernels of spgemmMasked (spgemm.hpp), which run when the
+// mask has no CSC to walk it by columns; otherwise the hash formulation
+// (kernels/spgemm_hash.cuh) runs.
+//
+// Reference: the reference's spgemmMaskedKernel, kernels/spgemm.hpp:17-79 — one
+// warp per mask row, every lane binary-searches A(i,:)'s columns in B(:,j) for each
+// mask entry.  Here: one thread per mask entry walks the SHORTER of the two sorted
+// lists and searches the longer one; entries whose lists are both long are
+// deferred to a warp each (spgemmMaskedHeavyKernel).
 #ifndef GRAPHBLAS_BACKEND_CUDA_KERNELS_SPGEMM_MASKED_CUH_
 #define GRAPHBLAS_BACKEND_CUDA_KERNELS_SPGEMM_MASKED_CUH_
 
@@ -15,79 +19,7 @@ namespace graphblas {
 namespace backend {
 
 #define GB_SPGEMM_NT 256
-#define GB_SPGEMM_ROWS_PER_GRAB 4
 #define GB_SPGEMM_HEAVY 32        // shorter list longer than this: warp per entry
-
-template <typename c, typename a, typename b, typename m,
-          typename MulOp, typename AddOp>
-__global__ void __launch_bounds__(GB_SPGEMM_NT)
-spgemmMaskedKernel(c* __restrict__           C_val,
-                   const Index* __restrict__ mask_rowptr,
-                   const Index* __restrict__ mask_colind,
-                   const m* __restrict__     mask_val,
-                   MulOp                     mul_op,
-                   AddOp                     add_op,
-                   c                         identity,
-                   const Index* __restrict__ A_rowptr,
-                   const Index* __restrict__ A_colind,
-                   const a* __restrict__     A_val,
-                   const Index* __restrict__ B_colptr,
-                   const Index* __restrict__ B_rowind,
-                   const b* __restrict__     B_val,
-                   Index                     nrows,
-                   unsigned long long*       work_counter,
-                   unsigned long long*       list_bytes) {
-  const int lane = threadIdx.x & 31;
-  unsigned long long scanned = 0;   // lane 0: entries of both lists per mask nnz
-  while (true) {
-    unsigned long long grab = 0;
-    if (lane == 0)
-      grab = atomicAdd(work_counter,
-                       static_cast<unsigned long long>(GB_SPGEMM_ROWS_PER_GRAB));
-    grab = __shfl_sync(GB_FULL_MASK, grab, 0);
-    if (grab >= static_cast<unsigned long long>(nrows)) break;
-    Index row_end_grab = static_cast<Index>(grab) + GB_SPGEMM_ROWS_PER_GRAB;
-    if (row_end_grab > nrows) row_end_grab = nrows;
-
-    for (Index row = static_cast<Index>(grab); row < row_end_grab; ++row) {
-      const Index m_beg = mask_rowptr[row];
-      const Index m_end = mask_rowptr[row + 1];
-      const Index a_beg = A_rowptr[row];
-      const Index a_end = A_rowptr[row + 1];
-      const Index a_len = a_end - a_beg;
-
-      for (Index edge = m_beg; edge < m_end; ++edge) {
-        c accumulator = identity;
-        if (mask_val[edge]) {
-          const Index j     = mask_colind[edge];
-          const Index b_beg = B_colptr[j];
-          const Index b_end = B_colptr[j + 1];
-          const Index b_len = b_end - b_beg;
-          scanned += static_cast<unsigned long long>(a_len + b_len);
-          if (a_len <= b_len) {
-            for (Index p = a_beg + lane; p < a_end; p += 32) {
-              const Index key = __ldg(A_colind + p);
-              const Index q = findSorted(B_rowind, b_beg, b_end, key);
-              if (q < b_end && __ldg(B_rowind + q) == key)
-                accumulator = add_op(mul_op(A_val[p], B_val[q]), accumulator);
-            }
-          } else {
-            for (Index q = b_beg + lane; q < b_end; q += 32) {
-              const Index key = __ldg(B_rowind + q);
-              const Index p = findSorted(A_colind, a_beg, a_end, key);
-              if (p < a_end && __ldg(A_colind + p) == key)
-                accumulator = add_op(mul_op(A_val[p], B_val[q]), accumulator);
-            }
-          }
-          accumulator = warpReduce(accumulator, add_op);
-        }
-        if (lane == 0) C_val[edge] = accumulator;
-      }
-    }
-  }
-  if (lane == 0 && scanned && list_bytes != NULL)
-    atomicAdd(list_bytes, 4ull*scanned);
-}
 
 // Edge-parallel form: one THREAD per mask entry (grid-stride).  In the triangle
 // count both operands are rows of L = tril(A): a high-id vertex next to many hubs

@@ -22,8 +22,7 @@ template <typename T, typename MonoidT>
 Info reduceFold(T* val, MonoidT op, T* partials, int grid) {
   T* d_out = partials + grid;
   cudaStream_t s = gbStream();
-  static const bool use_mail = getEnv("GB200_MAILBOX", 1) != 0;
-  const bool mail = use_mail && sizeof(T) == 4;
+  const bool mail = sizeof(T) == 4;
   const unsigned long long ticket = mail ? runtime().mailTicket() : 0ull;
   reduceFinalKernel<<<1, GB_REDUCE_NT, 0, s>>>(d_out, partials, grid, op,
       static_cast<T>(op.identity()), mail ? runtime().mailSlot(2) : NULL, ticket);

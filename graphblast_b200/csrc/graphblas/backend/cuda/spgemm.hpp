@@ -124,76 +124,65 @@ Info spgemmMasked(SparseMatrix<c>* C, const Matrix<m>* mask, BinaryOpT accum,
         prof_cell = profiler().d_cells + GB_PROF_SPGEMM;
       }
       profiler().begin(GB_PROF_SPGEMM, s);
-      // GB200_SPGEMM_ROWS=1 selects the warp-per-mask-row form (the reference's
-      // work decomposition) for comparison.
-      static const bool row_form = getEnv("GB200_SPGEMM_ROWS", 0) != 0;
-      if (row_form)
-        spgemmMaskedKernel<<<grid, GB_SPGEMM_NT, 0, s>>>(C->d_csrVal_,
+      // Hash formulation (kernels/spgemm_hash.cuh) when the mask can also be walked
+      // by columns; otherwise the search kernels.  A symmetric matrix borrows its
+      // CSR arrays for the column side, which is right only for the whole
+      // pattern — tril drops the flag.
+      static const bool hash_on = getEnv("GB200_SPGEMM_HASH", 1) != 0;
+      const bool mask_by_cols = sparse_mask->format_ == GrB_SPARSE_MATRIX_CSRCSC &&
+          sparse_mask->d_cscColPtr_ != NULL && sparse_mask->d_cscRowInd_ != NULL &&
+          sparse_mask->d_cscVal_ != NULL;
+      const Index B_ncols = use_tran_B ? B->nrows_ : B->ncols_;
+      const bool hashed = hash_on && mask_by_cols &&
+          sparse_mask->nrows_ == A_nrows && sparse_mask->ncols_ == B_ncols;
+      if (hashed) {
+        // work items per class: at most one partial chunk per owner plus the full ones
+        const size_t stride = static_cast<size_t>(A_nrows > B_ncols ? A_nrows : B_ncols) +
+            static_cast<size_t>(sparse_mask->nvals_)/GB_HASH_CHUNK_S + 1;
+        const size_t list_ints = 2*2*GB_HASH_NCLASS*stride;
+        Index* arena = reinterpret_cast<Index*>(desc->scratch(GB_SCRATCH_VEC_A,
+            (list_ints + 32)*sizeof(Index)));
+        HashItem* lists = reinterpret_cast<HashItem*>(arena);
+        unsigned int* cells = reinterpret_cast<unsigned int*>(arena + list_ints);
+        // cells: [0..2] item counts of pass 1, [4..6] of pass 2, [8..10] and
+        // [12..14] the grab counters
+        CUDA_CALL(cudaMemsetAsync(cells, 0, 32*sizeof(unsigned int), s));
+        spgemmHashClassifyKernel<<<gridFor(A_nrows, 256), 256, 0, s>>>(A_csrRowPtr,
+            sparse_mask->d_csrRowPtr_, A_nrows, false, lists, stride, cells);
+        GB_KERNEL_CHECK();
+        spgemmHashClassifyKernel<<<gridFor(B_ncols, 256), 256, 0, s>>>(B_cscColPtr,
+            sparse_mask->d_cscColPtr_, B_ncols, true,
+            lists + GB_HASH_NCLASS*stride, stride, cells + 4);
+        GB_KERNEL_CHECK();
+        CHECK((spgemmHashPass<false>(C->d_csrVal_, lists, stride, cells, cells + 8,
+            A_csrRowPtr, A_csrColInd, A_csrVal, B_cscColPtr, B_cscRowInd, B_cscVal,
+            sparse_mask->d_csrRowPtr_, sparse_mask->d_csrColInd_,
+            sparse_mask->d_csrVal_, sparse_mask->d_csrRowPtr_,
+            sparse_mask->d_csrColInd_, extractMul(op), extractAdd(op),
+            static_cast<c>(op.identity()), prof_cell, s)));
+        CHECK((spgemmHashPass<true>(C->d_csrVal_, lists + GB_HASH_NCLASS*stride,
+            stride, cells + 4, cells + 12,
+            B_cscColPtr, B_cscRowInd, B_cscVal, A_csrRowPtr, A_csrColInd, A_csrVal,
+            sparse_mask->d_cscColPtr_, sparse_mask->d_cscRowInd_,
+            sparse_mask->d_cscVal_, sparse_mask->d_csrRowPtr_,
+            sparse_mask->d_csrColInd_, extractMul(op), extractAdd(op),
+            static_cast<c>(op.identity()), prof_cell, s)));
+      } else {
+        // thread per mask entry; entries whose lists are both long are deferred
+        // to a warp-per-entry kernel through a device-side list (`work` counts it)
+        Index* heavy = reinterpret_cast<Index*>(desc->scratch(GB_SCRATCH_VEC_A,
+            2*static_cast<size_t>(sparse_mask->nvals_ + 1)*sizeof(Index)));
+        spgemmMaskedEdgeKernel<<<grid, GB_SPGEMM_NT, 0, s>>>(C->d_csrVal_,
             sparse_mask->d_csrRowPtr_, sparse_mask->d_csrColInd_,
             sparse_mask->d_csrVal_, extractMul(op), extractAdd(op),
             static_cast<c>(op.identity()), A_csrRowPtr, A_csrColInd, A_csrVal,
-            B_cscColPtr, B_cscRowInd, B_cscVal, A_nrows, work, prof_cell);
-      else {
-        // Hash formulation (kernels/spgemm_hash.cuh) when the mask can also be walked
-        // by columns; otherwise the search kernels.  A symmetric matrix borrows its
-        // CSR arrays for the column side, which is right only for the whole
-        // pattern — tril drops the flag.
-        static const bool hash_on = getEnv("GB200_SPGEMM_HASH", 1) != 0;
-        const bool mask_by_cols = sparse_mask->format_ == GrB_SPARSE_MATRIX_CSRCSC &&
-            sparse_mask->d_cscColPtr_ != NULL && sparse_mask->d_cscRowInd_ != NULL &&
-            sparse_mask->d_cscVal_ != NULL;
-        const Index B_ncols = use_tran_B ? B->nrows_ : B->ncols_;
-        const bool hashed = hash_on && mask_by_cols &&
-            sparse_mask->nrows_ == A_nrows && sparse_mask->ncols_ == B_ncols;
-        if (hashed) {
-          // work items per class: at most one partial chunk per owner plus the full ones
-          const size_t stride = static_cast<size_t>(A_nrows > B_ncols ? A_nrows : B_ncols) +
-              static_cast<size_t>(sparse_mask->nvals_)/GB_HASH_CHUNK_S + 1;
-          const size_t list_ints = 2*2*GB_HASH_NCLASS*stride;
-          Index* arena = reinterpret_cast<Index*>(desc->scratch(GB_SCRATCH_VEC_A,
-              (list_ints + 32)*sizeof(Index)));
-          HashItem* lists = reinterpret_cast<HashItem*>(arena);
-          unsigned int* cells = reinterpret_cast<unsigned int*>(arena + list_ints);
-          // cells: [0..2] item counts of pass 1, [4..6] of pass 2, [8..10] and
-          // [12..14] the grab counters
-          CUDA_CALL(cudaMemsetAsync(cells, 0, 32*sizeof(unsigned int), s));
-          spgemmHashClassifyKernel<<<gridFor(A_nrows, 256), 256, 0, s>>>(A_csrRowPtr,
-              sparse_mask->d_csrRowPtr_, A_nrows, false, lists, stride, cells);
-          GB_KERNEL_CHECK();
-          spgemmHashClassifyKernel<<<gridFor(B_ncols, 256), 256, 0, s>>>(B_cscColPtr,
-              sparse_mask->d_cscColPtr_, B_ncols, true,
-              lists + GB_HASH_NCLASS*stride, stride, cells + 4);
-          GB_KERNEL_CHECK();
-          CHECK((spgemmHashPass<false>(C->d_csrVal_, lists, stride, cells, cells + 8,
-              A_csrRowPtr, A_csrColInd, A_csrVal, B_cscColPtr, B_cscRowInd, B_cscVal,
-              sparse_mask->d_csrRowPtr_, sparse_mask->d_csrColInd_,
-              sparse_mask->d_csrVal_, sparse_mask->d_csrRowPtr_,
-              sparse_mask->d_csrColInd_, extractMul(op), extractAdd(op),
-              static_cast<c>(op.identity()), prof_cell, s)));
-          CHECK((spgemmHashPass<true>(C->d_csrVal_, lists + GB_HASH_NCLASS*stride,
-              stride, cells + 4, cells + 12,
-              B_cscColPtr, B_cscRowInd, B_cscVal, A_csrRowPtr, A_csrColInd, A_csrVal,
-              sparse_mask->d_cscColPtr_, sparse_mask->d_cscRowInd_,
-              sparse_mask->d_cscVal_, sparse_mask->d_csrRowPtr_,
-              sparse_mask->d_csrColInd_, extractMul(op), extractAdd(op),
-              static_cast<c>(op.identity()), prof_cell, s)));
-        } else {
-          // thread per mask entry; entries whose lists are both long are deferred
-          // to a warp-per-entry kernel through a device-side list (`work` counts it)
-          Index* heavy = reinterpret_cast<Index*>(desc->scratch(GB_SCRATCH_VEC_A,
-              2*static_cast<size_t>(sparse_mask->nvals_ + 1)*sizeof(Index)));
-          spgemmMaskedEdgeKernel<<<grid, GB_SPGEMM_NT, 0, s>>>(C->d_csrVal_,
-              sparse_mask->d_csrRowPtr_, sparse_mask->d_csrColInd_,
-              sparse_mask->d_csrVal_, extractMul(op), extractAdd(op),
-              static_cast<c>(op.identity()), A_csrRowPtr, A_csrColInd, A_csrVal,
-              B_cscColPtr, B_cscRowInd, B_cscVal, A_nrows, sparse_mask->nvals_,
-              heavy, work, prof_cell);
-          GB_KERNEL_CHECK();
-          spgemmMaskedHeavyKernel<<<grid, GB_SPGEMM_NT, 0, s>>>(C->d_csrVal_,
-              sparse_mask->d_csrColInd_, extractMul(op), extractAdd(op),
-              static_cast<c>(op.identity()), A_csrRowPtr, A_csrColInd, A_csrVal,
-              B_cscColPtr, B_cscRowInd, B_cscVal, heavy, work);
-        }
+            B_cscColPtr, B_cscRowInd, B_cscVal, A_nrows, sparse_mask->nvals_,
+            heavy, work, prof_cell);
+        GB_KERNEL_CHECK();
+        spgemmMaskedHeavyKernel<<<grid, GB_SPGEMM_NT, 0, s>>>(C->d_csrVal_,
+            sparse_mask->d_csrColInd_, extractMul(op), extractAdd(op),
+            static_cast<c>(op.identity()), A_csrRowPtr, A_csrColInd, A_csrVal,
+            B_cscColPtr, B_cscRowInd, B_cscVal, heavy, work);
       }
       GB_KERNEL_CHECK();
       profiler().end(GB_PROF_SPGEMM, s, 8.0*(A_nrows + 1) +

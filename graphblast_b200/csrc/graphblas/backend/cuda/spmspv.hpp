@@ -77,7 +77,7 @@ Info spmspvMerge(SparseVector<W>* w, const Vector<M>* mask, BinaryOpT accum,
     SemiringT op, const SparseMatrix<a>* A, const SparseVector<U>* u, Descriptor* desc,
     bool* prefer_pull = NULL) {
   // prefer_pull != NULL: the caller can still take the pull direction.  If the
-  // frontier's edges are more than GB200_EDGE_SWITCH_PCT percent of all stored entries the
+  // frontier's edges are more than 33 percent of all stored entries the
   // push is abandoned before it starts (*prefer_pull = true, w untouched): the
   // reference switches on the frontier's VERTEX share only (vector.hpp:318-342),
   // and a few hub vertices below that threshold can own most of the graph — at
@@ -160,9 +160,8 @@ Info spmspvMerge(SparseVector<W>* w, const Vector<M>* mask, BinaryOpT accum,
 
   // 1b) edge-based direction check (only for frontiers big enough to matter, so
   //     the small levels of a BFS pay nothing for it)
-  static const float edge_switch =
-      0.01f*static_cast<float>(getEnv("GB200_EDGE_SWITCH_PCT", 33));
-  if (prefer_pull != NULL && edge_switch > 0.f && nf >= 4096) {
+  const float edge_switch = 0.01f*33.f;     // share of the stored entries
+  if (prefer_pull != NULL && nf >= 4096) {
     const unsigned long long ticket = runtime().mailTicket();
     postIndexKernel<<<1, 1, 0, s>>>(offs + nf, runtime().mailSlot(4), ticket);
     GB_KERNEL_CHECK();

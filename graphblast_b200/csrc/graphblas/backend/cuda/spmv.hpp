@@ -52,10 +52,9 @@ Info spmvMergeLaunch(W* out, const Index* tile_rows, SemiringT op, const Index* 
         cudaFuncAttributePreferredSharedMemoryCarveout, GB_SPMV_CARVEOUT);
     configured = true;
   }
-  // 1 = 256-bit loads, 8 consecutive nonzeros per thread (needs 32-byte aligned
-  // arrays); 2 = 32-bit loads, lanes on consecutive nonzeros (any alignment).
-  static const int load_mode = getEnv("GB200_SPMV_LOADS", 1);
-  if ((load_mode == 2 || !aligned) && sizeof(a) == 4)
+  // 256-bit loads, 8 consecutive nonzeros per thread, where the arrays are 32-byte
+  // aligned; otherwise 32-bit loads, lanes on consecutive nonzeros.
+  if (!aligned && sizeof(a) == 4)
     spmvMergeKernelT<GB_SPMV_NT, GB_SPMV_IPT, false, true, true><<<nctas, GB_SPMV_NT, 0, s>>>(out, tile_rows, carry_row,
         carry_val, rowptr, colind, val, u, nrows, nnz, op.identity(),
         extractMul(op), extractAdd(op));
@@ -160,7 +159,6 @@ Info spmv(DenseVector<W>* w, const Vector<M>* mask, BinaryOpT accum, SemiringT o
       // assign() and this kernel itself, so inside a BFS no conversion pass runs;
       // a stale shadow costs one 4n-byte pass here.
       const bool bits_form = (op.identity() == static_cast<U>(0));
-      bool lazy_vals = false;
       unsigned long long mail_ticket = 0ull;
       double fixed_bytes;
       if (bits_form) {
@@ -178,12 +176,9 @@ Info spmv(DenseVector<W>* w, const Vector<M>* mask, BinaryOpT accum, SemiringT o
                                                    A_nrows);
         // The 0/1 result is published through the bitmap shadow only; the value
         // array is written when somebody asks for it (DenseVector::materialize).
-        static const bool eager = getEnv("GB200_EAGER_VALUES", 0) != 0;
-        W* w_out = eager ? w->d_val_ : static_cast<W*>(NULL);
-        lazy_vals = !eager;
-        static const bool use_mail = getEnv("GB200_MAILBOX", 1) != 0;
-        mail_ticket = use_mail ? runtime().mailTicket() : 0ull;
-        unsigned long long* mail = use_mail ? runtime().mailSlot(1) : NULL;
+        W* const w_out = NULL;
+        mail_ticket = runtime().mailTicket();
+        unsigned long long* mail = runtime().mailSlot(1);
         unsigned long long* done = desc->counters() + 4;
 #define GB_LAUNCH_PULL(SC, EE, OR)                                           \
         spmvMaskedOrPullBitsKernel<SC, EE, OR><<<grid, GB_PULL_NT, 0, s>>>(  \
@@ -208,7 +203,6 @@ Info spmv(DenseVector<W>* w, const Vector<M>* mask, BinaryOpT accum, SemiringT o
         // first-neighbour summary is colind[rowptr[row]]).  The kernel itself
         // moves fewer bytes (bitmaps, lazy values) — that is the saving.
         fixed_bytes = 12.0*A_nrows + 4.0;
-        (void)eager;
       } else {
         CHECK(mask->materialize());
         CHECK(u_t->materialize());
@@ -238,7 +232,7 @@ Info spmv(DenseVector<W>* w, const Vector<M>* mask, BinaryOpT accum, SemiringT o
       profiler().end(GB_PROF_PULL_BOOL, s, fixed_bytes);
       w->touched();
       w->bits_valid_ = bits_form;
-      w->vals_stale_ = lazy_vals;
+      w->vals_stale_ = bits_form;
       // The kernel wrote 0/1 and counted the ones: the next convert() or
       // a PlusMonoid reduce can reuse the count (one 8-byte read, no pass).
       w->count_pending_ = true;

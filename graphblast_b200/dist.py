@@ -237,8 +237,9 @@ class PeerExchange(object):
     """The library's own exchange (include/graphblast_b200.h, gb200_xchg_*): every
     rank maps every other rank's exchange block through CUDA IPC; the owner's
     kernel stores its frontier slice, count and epoch flag into all peers over
-    NVLink, and the level loop runs in C++ (gb200_dist_bfs).  torch.distributed
-    is used once, to pass the 64-byte IPC handles around."""
+    NVLink, and the whole traversal runs as one cooperative kernel per GPU
+    (gb200_dist_bfs_fused).  torch.distributed is used once, to pass the 64-byte
+    IPC handles around."""
 
     def __init__(self, gb, comm, device, offsets=None):
         """offsets: partition of the replicated array in 32-bit words; default =
@@ -274,12 +275,10 @@ class PeerExchange(object):
 
     def bfs(self, ops, n, source):
         levels = C.c_int(0)
-        import os
-        fused = os.environ.get("GB200_DIST_BFS_FUSED", "1") != "0"
-        fn = self.lib.gb200_dist_bfs_fused if fused else self.lib.gb200_dist_bfs
-        rc = fn(self._h, ops.v._h, ops.M._h, n, source, ops.desc._h, C.byref(levels))
+        rc = self.lib.gb200_dist_bfs_fused(self._h, ops.v._h, ops.M._h, n, source,
+                                           ops.desc._h, C.byref(levels))
         if rc != 0:
-            raise RuntimeError("gb200_dist_bfs%s failed: %d" % ("_fused" if fused else "", rc))
+            raise RuntimeError("gb200_dist_bfs_fused failed: %d" % rc)
         return levels.value
 
     def pr(self, p_own, M, n, alpha, eps, desc):
@@ -455,16 +454,14 @@ def bench_distributed(args, world, rank, local_rank):
     ops = GpuLocalOps(gb, n, lo, hi, rp_l, ci_l, colptr, rowind, desc)
     comm = Comm(bounds, dev)
 
-    # Exchange: the library's peer-memory path unless it cannot be set up (no
-    # IPC / peer access) or GB200_DIST_EXCHANGE=nccl asks for the NCCL baseline.
-    xchg = None
-    why = "requested"
-    if os.environ.get("GB200_DIST_EXCHANGE", "peer") == "peer":
-        try:
-            xchg = PeerExchange(gb, comm, dev)
-        except Exception as e:               # noqa: BLE001
-            why = str(e)
-            xchg = None
+    # Exchange: the library's peer-memory path unless it cannot be set up on some
+    # rank (no IPC / peer access); then every rank takes the NCCL all-gather path.
+    why = "failed on another rank"
+    try:
+        xchg = PeerExchange(gb, comm, dev)
+    except Exception as e:               # noqa: BLE001
+        why = str(e)
+        xchg = None
     agree = torch.tensor([1 if xchg is not None else 0], device=dev)
     dist.all_reduce(agree, op=dist.ReduceOp.MIN)
     if int(agree.item()) == 0:

@@ -300,16 +300,12 @@ int gb200_xchg_allgather_bits(gb200_xchg_t x, gb200_vector_t v,
                               long long* total_out);
 /* DEVICE pointer to the replicated bitmap of the last completed exchange. */
 int gb200_xchg_bits_ptr(gb200_xchg_t x, const uint32_t** d_bits);
-/* Level-synchronous BFS over the 1-D row partition with the level loop in the
- * library: v = levels of the owned vertices (length = owned rows of M), M = the
- * owned rows of A^T as an (owned x n) matrix with CSR and CSC.  Collective: every
- * rank calls it with the same n and source. */
-int gb200_dist_bfs(gb200_xchg_t x, gb200_vector_t v, gb200_matrix_t M,
-                   long long n, long long source, gb200_desc_t desc,
-                   int* levels_out);
-/* The same traversal as ONE persistent cooperative kernel per GPU: level loop,
- * direction decision, peer-memory exchange of the frontier slice and the cross-GPU
- * level barrier all on the device (csrc/dist_bfs_fused.cuh). */
+/* Level-synchronous BFS over the 1-D row partition as ONE persistent cooperative
+ * kernel per GPU: level loop, direction decision, peer-memory exchange of the
+ * frontier slice and the cross-GPU level barrier all on the device
+ * (csrc/dist_bfs_fused.cuh).  v_own = levels of the owned vertices (length = owned
+ * rows of M_local), M_local = the owned rows of A^T as an (owned x n) matrix with
+ * CSR and CSC.  Collective: every rank calls it with the same n and source. */
 int gb200_dist_bfs_fused(gb200_xchg_t x, gb200_vector_t v_own, gb200_matrix_t M_local,
                          long long n, long long source, gb200_desc_t desc,
                          int* levels_out);

@@ -1,6 +1,7 @@
-"""GPU tests of the multi-GPU layer: the peer-memory exchange and the native level
-loop (gb200_dist_bfs) against the oracle.  World size 1 runs on any GPU box (the
-owner stores into its own replica); the 2-rank test needs two GPUs."""
+"""GPU tests of the multi-GPU layer: the peer-memory exchange and the fused
+traversal kernel (gb200_dist_bfs_fused) against the oracle.  World size 1 runs on
+a single GPU (the owner stores into its own replica); the 2-rank test needs two
+GPUs."""
 import json
 import os
 import subprocess
